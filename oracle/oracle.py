@@ -3,9 +3,12 @@
 Imported only by tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs.
 The product package (dblink_b200/) never imports this module.
 """
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -23,7 +26,8 @@ c_dp = C.POINTER(C.c_double)
 
 def build(force=False, native=False):
     """liboracle.so (portable flags).  native=True: the -march=native build of the same sources, made on the machine
-    that runs it (bench.py's CPU legs); returns the portable library when that build is not possible."""
+    that runs it (bench.py's CPU legs) in a temporary directory removed at exit, so that nothing is written into a
+    tree that may be read-only; returns the portable library when that build is not possible."""
     so = os.path.join(_HERE, "liboracle.so")
     srcs = [os.path.join(_HERE, f) for f in ("dbl_oracle.c", "dbl_oracle.h", "dbl_oracle_priv.h", "dbl_refsweep.c", "Makefile")]
     srcs = [s for s in srcs if os.path.exists(s)]
@@ -31,8 +35,10 @@ def build(force=False, native=False):
         subprocess.run(["make", "-C", _HERE, "-s"], check=True)
     if native:
         try:
-            subprocess.run(["make", "-C", _HERE, "-s", "native"], check=True, capture_output=True)
-            nso = os.path.join(_HERE, "_native", "liboracle.so")
+            tmp = tempfile.mkdtemp(prefix="dbl_oracle_")
+            atexit.register(shutil.rmtree, tmp, True)  # a loaded library stays mapped after its file is removed
+            subprocess.run(["make", "-C", _HERE, "-s", "native", "NATIVE_DIR=" + tmp], check=True, capture_output=True)
+            nso = os.path.join(tmp, "liboracle.so")
             if os.path.exists(nso):
                 return nso
         except Exception:
@@ -51,7 +57,8 @@ def use_native():
 
 
 def flags():
-    return BUILD_FLAGS["native" if (_LIB is not None and "_native" in str(_LIB._name)) else "portable"]
+    native = _LIB is not None and _LIB._name != os.path.join(_HERE, "liboracle.so")
+    return BUILD_FLAGS["native" if native else "portable"]
 
 
 def lib():

@@ -147,3 +147,17 @@ def host_threads(cap=256):
         except Exception:
             pass
     return max(1, min(cap, n))
+
+
+def tree_files(root):
+    """Every file under the repository tree (but .git), with its size and mtime: taken before and after a run of
+    bench.py, which must write nothing into the tree (it may be read-only where the bench runs)."""
+    import os
+
+    out = {}
+    for dp, dirs, files in os.walk(root):
+        dirs[:] = [d for d in dirs if d != ".git"]
+        for f in files:
+            st = os.stat(os.path.join(dp, f))
+            out[os.path.relpath(os.path.join(dp, f), root)] = (st.st_size, st.st_mtime_ns)
+    return out

@@ -145,3 +145,43 @@ def test_baseline_config5_bit_parity_with_the_oracle(monkeypatch):
     d = _full_config_against_oracle(monkeypatch, 5, 1_000_000, 6, [4, 5, 6, 7, 8, 9], ("PCG-II", "PCG-I"))
     sizes = np.bincount(d["block"], minlength=64)
     assert sizes.max() > 1.3 * sizes.mean()  # the skew the configuration is about
+
+
+def test_bench_dump_outputs_follow_the_timed_steps(tmp_path):
+    """bench.py --dump-outputs: the state after warmup + steps sweeps, the same on a repeated run with the same
+    arguments (same inputs, same chain; the log-likelihood up to rounding), another one when --steps changes; nothing
+    written into the tree"""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    from helpers import tree_files
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+    def run(steps, name):
+        before = tree_files(root)
+        out = tmp_path / name
+        res = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--records", "20000", "--steps", str(steps),
+                              "--warmup", "2", "--no-cpu", "--no-small", "--no-e2e", "--dump-outputs", str(out)],
+                             capture_output=True, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr[-3000:]
+        assert tree_files(root) == before
+        line = json.loads(res.stdout.strip().splitlines()[-1])
+        assert line["steps"] == steps and line["state_hash_iteration"] == 2 + steps
+        dump = {p.name[:-4]: np.load(p) for p in out.iterdir()}
+        assert dump["iteration"][0] == 2 + steps and len(dump["link"]) == len(dump["record_ids"]) == 20000
+        assert all(a.dtype in (np.float32, np.float64) for a in dump.values())
+        return line["state_hash"], dump
+
+    h1, d1 = run(3, "a")
+    h2, d2 = run(3, "b")
+    h3, d3 = run(4, "c")
+    assert h1 == h2 and d1.keys() == d2.keys()
+    for k in d1:
+        if k == "log_likelihood":  # a sum of double atomics: its rounding depends on the order of the additions
+            np.testing.assert_allclose(d1[k], d2[k], rtol=1e-9)
+        else:
+            np.testing.assert_array_equal(d1[k], d2[k], err_msg=k)
+    assert h3 != h1 and not np.array_equal(d1["theta"], d3["theta"])

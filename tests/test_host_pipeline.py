@@ -197,20 +197,61 @@ def test_sampler_argument_checks():
 
 
 def test_bench_reference_arm_runs():
-    """`bench.py --impl reference` (the CPU arm the driver runs beside the GPU arm) prints one JSON line"""
+    """`bench.py --impl reference` (the CPU arm beside the GPU arm) prints one JSON line and writes nothing into the
+    tree (its -march=native oracle build goes to a temporary directory)"""
     import json
     import subprocess
     import sys
 
+    from helpers import tree_files
+
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     for sampler in ("PCG-II", "PCG-I"):
+        before = tree_files(root)
         res = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--records", "20000",
                               "--steps", "1", "--warmup", "0", "--cpu-sample", "500", "--sampler", sampler],
                              capture_output=True, text=True, timeout=600)
         assert res.returncode == 0, res.stderr[-2000:]
+        assert tree_files(root) == before
         line = json.loads(res.stdout.strip().splitlines()[-1])
         assert line["impl"] == "reference" and line["value"] > 0 and line["unit"] == "iterations/s"
         assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
+
+
+def test_bench_dump_outputs_sample_and_size(tmp_path):
+    """bench.py --dump-outputs on a state the size of the benchmark's: float32 / float64 files under 64 MB in all, the
+    same fixed rows on every call, values taken from those rows"""
+    import importlib.util
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    R, A, F = 1_000_000, 10, 2
+    rng = np.random.default_rng(3)
+    state = {"link": rng.integers(0, R, R, dtype=np.int32), "z": rng.integers(0, 2, (R, A), dtype=np.uint8),
+             "y": rng.integers(0, 50_000, (R, A), dtype=np.int32), "block": rng.integers(0, 64, R, dtype=np.int32),
+             "theta": rng.uniform(0, 1, (A, F))}
+    summary = {"agg_dist": rng.integers(0, R, (A, F)), "rec_dist": rng.integers(0, R, A + 1), "log_likelihood": -1.5e7,
+               "num_isolates": 12345, "iteration": 11}
+    dirs = [tmp_path / "a", tmp_path / "b"]
+    for d in dirs:
+        bench.dump_outputs(str(d), state, summary)
+    files = sorted(p.name for p in dirs[0].iterdir())
+    assert {"link.npy", "y.npy", "z.npy", "block.npy", "theta.npy", "record_ids.npy", "entity_ids.npy"} <= set(files)
+    assert sum((dirs[0] / f).stat().st_size for f in files) <= 64 << 20
+    for f in files:
+        a, b = np.load(dirs[0] / f), np.load(dirs[1] / f)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), f
+    out = {f[:-4]: np.load(dirs[0] / f) for f in files}
+    rec, ent = out["record_ids"].astype(np.int64), out["entity_ids"].astype(np.int64)
+    assert 100_000 < len(rec) < R and np.all(np.diff(rec) > 0) and np.all(np.diff(ent) > 0)
+    np.testing.assert_array_equal(out["link"], state["link"][rec])
+    np.testing.assert_array_equal(out["z"], state["z"][rec])
+    np.testing.assert_array_equal(out["y"], state["y"][ent])
+    np.testing.assert_array_equal(out["block"], state["block"][ent])
+    np.testing.assert_array_equal(out["theta"], state["theta"])
+    assert out["log_likelihood"][0] == -1.5e7 and out["iteration"][0] == 11
 
 
 def test_arrow_linkage_structure_equals_list_form(tmp_path):
