@@ -16,6 +16,7 @@
 #include <unistd.h>
 
 #include <algorithm>
+#include <cfloat>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -452,6 +453,90 @@ __device__ __forceinline__ bool in_support(const ValParams &p, const AttrDev &at
   return row_find(at, xr, v, e);
 }
 
+constexpr int VALUE_REDO = -2;  // what k_values stores for a draw it leaves to k_values_log
+// marks the running sweep for k_values_log in the control block (a word only these two kernels use; through the
+// RowSet's pointer, since one more kernel parameter alone changes the register allocation of k_values)
+__device__ __forceinline__ int redo_later(const ValParams &p, uint32_t iter) {
+  const_cast<long long *>(p.rows.ctl)[CTL_VALUES_REDO] = iter;
+  return VALUE_REDO;
+}
+
+// The mixture of GU:593-597 in the log domain (DESIGN.md 4.3), for the draws whose sum of perturbation weights is
+// not finite: a large cluster of agreeing records overflows prod_r g_r(v), and beyond the cached powers n(v)^k can
+// underflow to 0 / 0.  log b_k(v) = log probs(v) + k log n(v); log W(v) = log b_k(v) + log(G(v) - 1), or
+// log b_k(v) + sum_r log g_r(v) where G itself overflows.  The same candidates in the same order as value_update,
+// with det_log / det_exp, so the oracle draws the same value (oracle/dbl_oracle.c value_draw_log).
+__device__ __noinline__ int value_update_log(const ValParams &p, const AttrDev &at, int a, int lo, int hi, int k,
+                                             bool collapsed, U2 u) {
+  const int *rec = p.rec_by_ent;
+  const double kk = at.is_const ? 0.0 : (double)k;
+  auto lbase = [&](int v) { return det_log(at.probs[v]) + kk * det_log(at.norm[v]); };
+  double bmax = lbase(0), Z = 0.0;  // Z = sum_v b_k(v) / exp(bmax) over every value, in ascending id
+  for (int v = 1; v < at.V; ++v) {
+    const double l = lbase(v);
+    if (l > bmax) bmax = l;
+  }
+  for (int v = 0; v < at.V; ++v) Z += det_exp(lbase(v) - bmax);
+  // pass 0: max of log W; pass 1: sum of exp(log W - max); pass 2: the inverse CDF at u1
+  double lmax = 0.0, S = 0.0, target = 0.0, cum = 0.0;
+  bool any = false, base = false;
+  int picked = -1, last_pos = -1;
+  for (int pass = 0; pass < 3 && !base && picked < 0; ++pass) {
+    for (int i = lo; i < hi && picked < 0; ++i) {
+      const int xr = p.x[(int64_t)rec[i] * p.A + a];
+      if (xr < 0) continue;
+      bool repeated = false;  // every value of this record's row has been seen (value_update)
+      for (int j = lo; j < i && !repeated; ++j) repeated = (p.x[(int64_t)rec[j] * p.A + a] == xr);
+      if (repeated) continue;
+      const int nv = at.is_const ? 1 : (at.rowptr[xr + 1] - at.rowptr[xr]);
+      for (int q = 0; q < nv && picked < 0; ++q) {
+        const int v = at.is_const ? xr : at.col[at.rowptr[xr] + q];
+        bool seen = false;
+        for (int j = lo; j < i && !seen; ++j) {
+          const int rj = rec[j];
+          if (p.x[(int64_t)rj * p.A + a] < 0) continue;
+          seen = in_support(p, at, a, rj, v);
+        }
+        if (seen) continue;
+        double G = 1.0, L = 0.0;
+        for (int j = i; j < hi; ++j) {
+          const int rj = rec[j];
+          if (p.x[(int64_t)rj * p.A + a] < 0) continue;
+          double g;
+          if (g_factor(p, at, a, rj, collapsed, v, g)) { G = G * g; L = L + det_log(g); }
+        }
+        if (!(G > 1.0)) continue;  // W(v) = 0
+        const double lw = lbase(v) + (G <= DBL_MAX ? det_log(G - 1.0) : L);
+        if (pass == 0) {
+          if (!any || lw > lmax) lmax = lw;
+          any = true;
+        } else if (pass == 1) {
+          S += det_exp(lw - lmax);
+        } else {
+          const double W = det_exp(lw - lmax);
+          cum += W;
+          if (W > 0.0) last_pos = v;
+          if (cum > target) picked = v;
+        }
+      }
+    }
+    if (pass == 0 && !any) base = true;
+    if (pass == 1) {  // P(base) = Z / (Z + sum W)  (GU:593-594)
+      const double d = (lmax + det_log(S)) - (bmax + det_log(Z));
+      base = u.u0 < 1.0 / (1.0 + det_exp(d));
+      target = u.u1 * S;
+    }
+  }
+  if (!base) return picked >= 0 ? picked : last_pos;
+  const double bt = u.u1 * Z;
+  double c = 0.0;
+  for (int v = 0; v < at.V; ++v) {
+    c += det_exp(lbase(v) - bmax);
+    if (c > bt) return v;
+  }
+  return at.V - 1;
+}
+
 // new value of attribute a of entity e.  UB > 1: the loop over the similarity row of a single linked record fetches
 // UB candidates at a time (independent loads, same sums in the same order): for problems too small to fill the GPU
 // the kernel's time is the longest dependent-load chain of one thread, not throughput
@@ -536,6 +621,7 @@ __device__ int value_update(const ValParams &p, uint32_t iter, int64_t e, int a)
         for (int i = 0; i < UB; ++i)
           if (q + i < nv) total += W[i];
       }
+      if (!isfinite(total)) return redo_later(p, iter);
       if (u.u0 < 1.0 / (1.0 + total)) return base_draw(b, u.u1);  // GU:593-594
       target = u.u1 * total;
       for (int q = 0; q < nv && picked < 0; q += UB) {
@@ -555,6 +641,7 @@ __device__ int value_update(const ValParams &p, uint32_t iter, int64_t e, int a)
         int v;
         total += weight(q, v);
       }
+      if (!isfinite(total)) return redo_later(p, iter);
       if (u.u0 < 1.0 / (1.0 + total)) return base_draw(b, u.u1);  // GU:593-594
       target = u.u1 * total;
       for (int q = 0; q < nv && picked < 0; ++q) {
@@ -622,6 +709,7 @@ __device__ int value_update(const ValParams &p, uint32_t iter, int64_t e, int a)
       }
     }
     if (pass == 0) {
+      if (!isfinite(total)) return redo_later(p, iter);
       if (u.u0 < 1.0 / (1.0 + total)) return base_draw(b, u.u1);  // GU:593-594
       target = u.u1 * total;
     }
@@ -642,6 +730,28 @@ __global__ void __launch_bounds__(128) k_values(ValParams p) {
     if (e < 0) continue;
     const int a = (int)(t % p.A);
     p.y[e * p.A + a] = value_update<UB>(p, iter, e, a);
+  }
+}
+
+// The draws k_values left (sum of the perturbation weights not finite), in the log domain.  A kernel of its own, so
+// that the rarely taken fallback costs k_values nothing (registers, stack): when no draw was left in this sweep every
+// block returns at once.
+__global__ void __launch_bounds__(128) k_values_log(ValParams p) {
+  if (p.rows.dead()) return;
+  const uint32_t iter = (uint32_t)(p.rows.ctl[CTL_ITER] + 1);
+  if (p.rows.ctl[CTL_VALUES_REDO] != (long long)iter) return;
+  const bool collapsed = (p.sampler == DBL_PCG_I || p.sampler == DBL_PCG_II);
+  const int64_t n = p.rows.count() * p.A;
+  GRID_STRIDE(t, n) {
+    const int64_t e = p.rows.row(t / p.A);
+    if (e < 0) continue;
+    const int a = (int)(t % p.A);
+    if (p.y[e * p.A + a] != VALUE_REDO) continue;
+    const int lo = p.ent_rec_ptr[e], hi = p.ent_rec_ptr[e + 1];
+    int k = 0;
+    for (int i = lo; i < hi; ++i) k += (p.x[(int64_t)p.rec_by_ent[i] * p.A + a] >= 0);
+    const U2 u = uniform2(p.seed, PH_VALUE, iter, (uint32_t)e, (uint32_t)a);
+    p.y[e * p.A + a] = value_update_log(p, p.attrs[a], a, lo, hi, k, collapsed, u);
   }
 }
 
@@ -2289,7 +2399,8 @@ static int update_owned(dbl_ctx *ctx, int sampler) {
   // latency-bound sizes (the grid does not fill the GPU a few times over): the variant with batched loads
   if (ctx->E * A <= (int64_t)ctx->sm_count * 2048 * 4) k_values<8><<<grid_rows(ctx->E * A, 128), 128, 0, ctx->stream>>>(vp);
   else k_values<DBL_VALUES_UB_LARGE><<<grid_rows(ctx->E * A, 128), 128, 0, ctx->stream>>>(vp);
-  ctx->launches += 1;
+  k_values_log<<<std::min(grid_rows(ctx->E * A, 128), ctx->sm_count * 4), 128, 0, ctx->stream>>>(vp);
+  ctx->launches += 2;
   // (4) N(e), new block ids, distortions, partial summary
   return refresh_summary(ctx, true);
 }
@@ -2584,7 +2695,7 @@ extern "C" int dbl_set_rebalance(dbl_ctx *ctx, int32_t period, double threshold)
 static int preload_kernels(dbl_ctx *ctx) {
   cudaFuncAttributes fa;
 #define DBL_LOAD(k) CUDA_TRY(cudaFuncGetAttributes(&fa, k))
-  DBL_LOAD(k_theta); DBL_LOAD(k_link_heavy); DBL_LOAD(k_commit_link_keys); DBL_LOAD(k_build_tiles); DBL_LOAD(k_values<DBL_VALUES_UB_LARGE>); DBL_LOAD(k_values<8>); DBL_LOAD(k_entity_post); DBL_LOAD(k_dist);
+  DBL_LOAD(k_theta); DBL_LOAD(k_link_heavy); DBL_LOAD(k_commit_link_keys); DBL_LOAD(k_build_tiles); DBL_LOAD(k_values<DBL_VALUES_UB_LARGE>); DBL_LOAD(k_values<8>); DBL_LOAD(k_values_log); DBL_LOAD(k_entity_post); DBL_LOAD(k_dist);
   DBL_LOAD(k_reduce_local); DBL_LOAD(k_finish); DBL_LOAD(k_move_ent); DBL_LOAD(k_move_rec); DBL_LOAD(k_publish_barrier);
   DBL_LOAD(k_unpack_ent_p2p); DBL_LOAD(k_unpack_rec_p2p); DBL_LOAD(k_reduce_peers); DBL_LOAD(k_lpt);
   DBL_LOAD(k_link_generic); DBL_LOAD(k_link_match); DBL_LOAD(k_link_pruned); DBL_LOAD(k_state_hash);

@@ -65,6 +65,7 @@ enum : int {
   CTL_REPLACED = 8,   // block -> rank placements adopted by the device-side LPT
   CTL_WORK = 9,       // work counter of the persistent link kernel
   CTL_HEAVY = 10,     // records the pruned link kernel handed to k_link_heavy in the running sweep
+  CTL_VALUES_REDO = 11,  // iteration of the last sweep in which k_values left a draw to k_values_log
   CTL_WORDS = 16
 };
 constexpr long long ST_ZERO_MASS = 1, ST_PEER_TIMEOUT = 2, ST_PEER_ERROR = 4;

@@ -12,6 +12,7 @@
 #include "dbl_oracle.h"
 #include "dbl_oracle_priv.h"
 
+#include <float.h>
 #include <math.h>
 #include <pthread.h>
 #include <stdio.h>
@@ -1078,6 +1079,57 @@ static int in_support(const orc_state *s, int64_t r, int a, int v) {
   return row_find(ix, xr, v, &e);
 }
 
+/* The mixture of GU:593-597 in the log domain (DESIGN.md 4.3), for the draws whose sum of perturbation weights is not
+   finite (a large cluster of agreeing records overflows prod_r g_r(v); beyond the cached powers n(v)^k can underflow):
+   log b_k(v) = log probs(v) + k log n(v), log W(v) = log b_k(v) + log(G(v) - 1), or + sum_r log g_r(v) where G
+   overflows.  Same candidates, same order and the same det_log / det_exp operations as value_update_log of the
+   engine (dblink_b200/csrc/dbl_engine.cu). */
+static double lbase_of(const orc_index *ix, double kk, int v) { return orc_det_log(ix->probs[v]) + kk * orc_det_log(ix->norm[v]); }
+static int value_draw_log(const orc_state *s, const int64_t *obs, int64_t k, int a, int collapsed, double u0, double u1) {
+  const orc_index *ix = s->m->idx[a];
+  const double kk = ix->is_const ? 0.0 : (double)k;
+  double bmax = lbase_of(ix, kk, 0), Z = 0.0;
+  for (int v = 1; v < ix->V; ++v) { double l = lbase_of(ix, kk, v); if (l > bmax) bmax = l; }
+  for (int v = 0; v < ix->V; ++v) Z += orc_det_exp(lbase_of(ix, kk, v) - bmax);
+  double lmax = 0.0, S = 0.0, target = 0.0, cum = 0.0;
+  int any = 0, base = 0, picked = -1, last_pos = -1;
+  for (int pass = 0; pass < 3 && !base && picked < 0; ++pass) {
+    for (int64_t i = 0; i < k && picked < 0; ++i) {
+      const int32_t *vals; int32_t single;
+      int nv = support_of(s, obs[i], a, &vals, &single);
+      for (int q = 0; q < nv && picked < 0; ++q) {
+        int v = vals[q];
+        int seen = 0;
+        for (int64_t j = 0; j < i && !seen; ++j) seen = in_support(s, obs[j], a, v);
+        if (seen) continue;
+        double G = 1.0, L = 0.0;
+        for (int64_t j = i; j < k; ++j) { double g; if (g_factor(s, obs[j], a, collapsed, v, &g)) { G = G * g; L = L + orc_det_log(g); } }
+        if (!(G > 1.0)) continue; /* W(v) = 0 */
+        const double lw = lbase_of(ix, kk, v) + (G <= DBL_MAX ? orc_det_log(G - 1.0) : L);
+        if (pass == 0) { if (!any || lw > lmax) lmax = lw; any = 1; }
+        else if (pass == 1) S += orc_det_exp(lw - lmax);
+        else {
+          const double W = orc_det_exp(lw - lmax);
+          cum += W;
+          if (W > 0.0) last_pos = v;
+          if (cum > target) picked = v;
+        }
+      }
+    }
+    if (pass == 0 && !any) base = 1;
+    if (pass == 1) { /* P(base) = Z / (Z + sum W) (GU:593-594) */
+      const double d = (lmax + orc_det_log(S)) - (bmax + orc_det_log(Z));
+      base = u0 < 1.0 / (1.0 + orc_det_exp(d));
+      target = u1 * S;
+    }
+  }
+  if (!base) return picked >= 0 ? picked : last_pos;
+  const double bt = u1 * Z;
+  double c = 0.0;
+  for (int v = 0; v < ix->V; ++v) { c += orc_det_exp(lbase_of(ix, kk, v) - bmax); if (c > bt) return v; }
+  return ix->V - 1;
+}
+
 /* Protocol draw of y_{e,a}: updateEntityValueCollapsed GU:576-599 / updateEntityValue GU:605-646.
    lrec = linked records (ascending id), nl = their count. */
 static int value_draw(const orc_state *s, const int64_t *lrec, int64_t nl, int a, int sampler, double u0, double u1) {
@@ -1123,6 +1175,7 @@ static int value_draw(const orc_state *s, const int64_t *lrec, int64_t nl, int a
       }
     }
     if (pass == 0) {
+      if (!isfinite(total)) { result = value_draw_log(s, obs, k, a, collapsed, u0, u1); free(obs); return result; }
       if (u0 < 1.0 / (1.0 + total)) { result = base_draw(&b, u1); free(obs); return result; } /* GU:593-594 */
       target = u1 * total;
     }
@@ -1155,23 +1208,26 @@ void orc_ref_value_pmf(const orc_state *s, int64_t e, int a, int sampler, double
   for (int64_t i = 0; i < nl; ++i) if (s->x[rec[ptr[e] + i] * A + a] >= 0) obs[k++] = rec[ptr[e] + i];
   int forced = -1;
   if (!collapsed) for (int64_t i = 0; i < k && forced < 0; ++i) if (!s->z[obs[i] * A + a]) forced = s->x[obs[i] * A + a];
-  double z = 0.0;
+  /* log p(v), then exp(log p - max): a large cluster overflows the product of its factors */
+  double lmax = -HUGE_VAL, z = 0.0;
   for (int v = 0; v < V; ++v) {
-    double p;
-    if (forced >= 0) p = (v == forced) ? 1.0 : 0.0;
-    else if (k == 0 || (!collapsed && ix->is_const)) p = ix->phi[v];
+    double lp;
+    if (forced >= 0) lp = (v == forced) ? 0.0 : -HUGE_VAL;
+    else if (k == 0 || (!collapsed && ix->is_const)) lp = log(ix->phi[v]);
     else if (sampler == ORC_GIBBS_SEQ) {
-      p = ix->phi[v];
+      lp = log(ix->phi[v]);
       for (int64_t i = 0; i < k; ++i) { /* GU:689 */
         int32_t xr = s->x[obs[i] * A + a];
-        p *= orc_index_exp_sim_of(ix, xr, v) * ix->norm[v] * ix->phi[xr];
+        lp += log(orc_index_exp_sim_of(ix, xr, v) * ix->norm[v] * ix->phi[xr]);
       }
     } else {
-      p = ix->probs[v] * (ix->is_const ? 1.0 : pow(ix->norm[v], (double)k));
-      for (int64_t i = 0; i < k; ++i) { double g; if (g_factor(s, obs[i], a, collapsed, v, &g)) p *= g; }
+      lp = log(ix->probs[v]) + (ix->is_const ? 0.0 : (double)k * log(ix->norm[v]));
+      for (int64_t i = 0; i < k; ++i) { double g; if (g_factor(s, obs[i], a, collapsed, v, &g)) lp += log(g); }
     }
-    pmf[v] = p; z += p;
+    pmf[v] = lp;
+    if (lp > lmax) lmax = lp;
   }
+  for (int v = 0; v < V; ++v) { pmf[v] = exp(pmf[v] - lmax); z += pmf[v]; }
   for (int v = 0; v < V; ++v) pmf[v] /= z;
   free(obs); free(ptr); free(rec);
 }

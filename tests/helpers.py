@@ -161,3 +161,22 @@ def tree_files(root):
             st = os.stat(os.path.join(dp, f))
             out[os.path.relpath(os.path.join(dp, f), root)] = (st.st_size, st.st_mtime_ns)
     return out
+
+
+def agreeing_cluster(rng, x, y, link, z, K, distorted=(), flag_rate=0.0):
+    """A valid state in which records 0..K-1 all copy record 0 and link to entity 0, whose values are theirs: a
+    cluster of K agreeing records, built on the state (y, link, z) of the records x.  The cluster's flags are 1 on
+    the attributes in `distorted` and 0 elsewhere; every other flag is set to 1 with probability flag_rate (a valid
+    change at any rate) so that the next theta draw lands near flag_rate.  -> x, y, link, z"""
+    x, y, link, z = (np.array(t, copy=True) for t in (x, y, link, z))
+    x[:K] = x[0]
+    link[:K] = 0
+    y[0] = np.where(x[0] >= 0, x[0], y[0])
+    z[:K] = 0
+    for a in distorted:
+        z[:K, a] = 1
+    z[K:] |= (rng.random(z[K:].shape) < flag_rate).astype(z.dtype)
+    obs = x >= 0
+    z |= (obs & (x != y[link])).astype(z.dtype)  # records of entity 0 outside the cluster
+    z[:K][~obs[:K]] = 1
+    return x, y, link, z
